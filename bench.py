@@ -2,7 +2,7 @@
 """bench.py — learner tokens processed/sec (GRPO step, Qwen2.5-7B LoRA) on B200.
 
 Contract: python bench.py --gpus N --steps K --warmup W [--impl reference] [--config cfg2|cfg3|cfg4|cfg5]
-  (N > 1: launched by torch.distributed.run, one rank per GPU).
+  [--dump-outputs DIR]  (N > 1: launched by torch.distributed.run, one rank per GPU).
 
 Workloads (BASELINE.json configs; SURVEY.md 8d):
   cfg2 (default, the headline): GRPO learner, Qwen2.5-7B-shaped random-init NF4 base + rank-16 LoRA, group_size 8,
@@ -226,6 +226,19 @@ class CpuArm:
         return tok_s, desc, t_step
 
 
+DUMP_SAMPLE = 1 << 22   # positions kept per flat LoRA-sized buffer: 3 x 16 MB of float32
+
+
+def step_outputs(pol):
+    """What the last learner step hands its caller: the loss (sum over the micro-batches, float64) and the updated adapter,
+    plus the Adam moments, which carry that step's gradient (the optimizer step zeroes the gradient buffer itself).  The
+    flat buffers hold ~40M values at the Qwen2.5-7B shape, so a fixed sample of DUMP_SAMPLE positions (seed 0) is kept."""
+    n = pol.lora_flat.numel()
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values.to(pol.device)
+    out = {"loss": pol.loss_accum, "lora": pol.lora_flat[idx], "adam_m": pol.adam_m[idx], "adam_v": pol.adam_v[idx]}
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
 def config_dict(args):
     preset = PRESETS.get(args.config)
     if args.config == "cfg2":
@@ -382,7 +395,11 @@ def main():
                     help="NF4 base: resident bf16 cache (auto/cache), dequant into a scratch before each GEMM, or inside the GEMM mainloop")
     ap.add_argument("--lean", action="store_true", help="long configs (cfg4): one e2e warm-up, no repeat of the device timing, one exchange-timing step")
     ap.add_argument("--no_verify_exchange", action="store_true", help="N > 1: skip the post-run parameter identity / NCCL cross-check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (see step_outputs) as DIR/<name>.npy; --impl b200, one GPU")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b200 and --gpus 1")
     preset = PRESETS[args.config]
     if args.new_tokens is None:
         args.new_tokens = preset["T"]
@@ -583,6 +600,10 @@ def main():
         torch.cuda.profiler.stop()
         return
     ms_dev, clocks, launches = timed(device_step, args.steps, sample_clocks=True)
+    if args.dump_outputs:   # before the e2e and diagnostic steps below move the adapter on
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in step_outputs(pol).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     for _ in range(1 if args.lean else 2):
         e2e_step()
     ms_e2e, _, _ = timed(e2e_step, args.steps)

@@ -21,6 +21,7 @@ What is NOT pinned by the reference (arithmetic lives in un-vendored dependencie
 """
 from __future__ import annotations
 
+import hashlib
 import math
 from dataclasses import dataclass
 
@@ -349,6 +350,19 @@ def make_params(cfg: OracleConfig, seed=0, quantize_base=True, lora_b_std=0.01, 
         params[f"l{i}.ln1"] = (1 + 0.1 * torch.randn(H, generator=g)).to(torch.bfloat16).float().to(device)
         params[f"l{i}.ln2"] = (1 + 0.1 * torch.randn(H, generator=g)).to(torch.bfloat16).float().to(device)
     return params, nf4
+
+
+def params_digest(params, nf4):
+    """sha256 over every parameter (fp32 bytes) and NF4 code / scale array of make_params' output, in name order."""
+    h = hashlib.sha256()
+    for k in sorted(params):
+        h.update(k.encode())
+        h.update(params[k].detach().cpu().float().numpy().tobytes())
+    for k in sorted(nf4):
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(nf4[k][0]).tobytes())
+        h.update(np.ascontiguousarray(nf4[k][1]).tobytes())
+    return h.hexdigest()
 
 
 def make_batch(cfg: OracleConfig, n_seq, P, T, seed=0, ragged=True, group_size=None, learner="grpo"):

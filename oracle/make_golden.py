@@ -225,7 +225,8 @@ def main():
     cfg = lo.OracleConfig(vocab=512, hidden=128, inter=256, n_layers=2, n_q_heads=4, n_kv_heads=2, head_dim=32,
                           lora_r=16, lora_alpha=16)
     P, T, B = 16, 32, 2
-    params, nf4 = lo.make_params(cfg, seed=1234)
+    seed = 1234
+    params, nf4 = lo.make_params(cfg, seed=seed)
     prompts, answers, _ = lo.make_batch(cfg, 4, P, T, seed=1, ragged=True)
     rewards = np.array([1.1, 0.1, 0.2, 1.0])  # summed (format+accuracy) rewards of one group of 4
     baseline = rewards.mean()
@@ -235,11 +236,10 @@ def main():
     for i, (p, a) in enumerate(zip(prompts, answers)):
         fixtures[f"prompt{i}"] = np.array(p)
         fixtures[f"answer{i}"] = np.array(a)
-    for k, v in params.items():
-        fixtures["param." + k] = v.detach().numpy()
-    for k, (packed, absmax) in nf4.items():
-        fixtures["nf4p." + k] = packed
-        fixtures["nf4a." + k] = absmax
+    # the parameters are not stored (they would more than double the file): the loader regenerates them from the seed
+    # and checks them against this digest
+    fixtures["param_seed"] = np.int64(seed)
+    fixtures["param_sha256"] = np.array(lo.params_digest(params, nf4))
 
     for mode in ("fp32", "bf16"):
         ctx = None
@@ -278,11 +278,15 @@ def main():
                 g2, _ = ln._compute_gradients(prompts[2:], answers[2:], r[2:])
                 ln.optimizer.zero_grad()
                 ln.apply_merged_gradients([g1, g2])  # REFERENCE CODE (:302-333) with Adam8bit -> torch Adam
+                # stored as the fp32 update (new - old), which compresses better and adds back to the new value exactly
                 sd = dict(ln.policy.named_parameters())
                 for i in range(cfg.n_layers):
                     for m in lo.LORA_MODULES:
                         for ab in ("A", "B"):
-                            fixtures[f"fp32.merged_step.l{i}.{m}.{ab}"] = sd[hf_grad_name(i, m, ab)].detach().numpy().copy()
+                            new = sd[hf_grad_name(i, m, ab)].detach().numpy()
+                            old = params[f"l{i}.{m}.{ab}"].detach().numpy()
+                            assert np.array_equal(old + (new - old), new)
+                            fixtures[f"fp32.merged_update.l{i}.{m}.{ab}"] = new - old
             if mode == "fp32" and kind == "grpo":
                 # quirk Q1: a micro-batch containing an exact-zero reward is skipped (:459)
                 rq = [0.5, 0.0, -0.25, 1.0]
