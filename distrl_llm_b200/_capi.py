@@ -31,6 +31,10 @@ class LossArgs(C.Structure):
                 ("ref_lp", c_void_p), ("kl_beta", C.c_double), ("old_lp", c_void_p), ("clip_eps", C.c_double)]
 
 
+class EntropyArgs(C.Structure):
+    _fields_ = [("alpha", C.c_double), ("ent_out", c_void_p), ("ent_accum", c_void_p)]
+
+
 class LayerWeights(C.Structure):
     _fields_ = [
         ("qkv_packed", c_void_p), ("qkv_absmax", c_void_p),
@@ -132,6 +136,14 @@ SIGNATURES = {
     "b200rl_model_pass": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                   c_void_p, c_void_p]),
     "b200rl_model_pass_packed": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "b200rl_logprob_entropy": (c_int, [c_void_p, c_ll, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, C.c_double, c_void_p,
+                                       c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, C.c_double,
+                                       c_void_p, c_void_p]),
+    "b200rl_loss_value_entropy": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, C.c_double, c_void_p, C.c_double, c_void_p,
+                                          c_int, c_int, c_int, c_void_p, C.c_double, c_void_p, c_void_p]),
+    "b200rl_model_pass_ent": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                      c_int, c_void_p, c_void_p, c_void_p]),
+    "b200rl_model_pass_packed_ent": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "b200rl_model_microbatch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
 }

@@ -19,20 +19,44 @@ namespace b200rl {
 static constexpr float LOG2E = 1.4426950408889634f;
 static constexpr float LN2 = 0.6931471805599453f;
 
+// Optional per-token entropy (ENT = true; reference helper BaseLearner.compute_entropy_bonus, distributed_actor.py:266-281,
+// whose call sites are commented out at :377-379 and :472-480):
+//   H = -sum_v p_v ln p_v,  p = softmax(z) at temperature 1, fp32.
+// Pass 1 carries a third running quantity next to (m, s) in the log2 domain, shifted by the running max m:
+//   u = sum_v 2^(y_v - m) (y_v - m),  y = z log2(e);  when m moves to m' > m:  u' = 2^(m - m') (u + s (m - m')).
+// Then H = ln2 (log2 s - u / s), which stays accurate on peaked rows (lse - E[z] cancels there).
+// Pass 2 adds the gradient of the bonus term -e * H, e = alpha * mask / (len * Bm * nb):
+//   d(-e H)/dz_v = e p_v (ln p_v + H),  ln p_v = (y_v - lse2) ln2 (no extra exp / log).
+// merge (om, os, ou) into (m, s, u); nm = max(m, om).  A side with s == 0 (m == -inf) contributes nothing.
+__device__ __forceinline__ void ent_combine(float m, float s, float& u, float om, float os, float ou, float nm) {
+  const float a = s > 0.f ? exp2f(m - nm) * (u + s * (m - nm)) : 0.f;
+  const float b = os > 0.f ? exp2f(om - nm) * (ou + os * (om - nm)) : 0.f;
+  u = a + b;
+}
+
+struct EntArgs {
+  const int* mask;   // [Bm*T] answer mask; e = 0 where it is 0
+  const int* lens;   // [Bm] answer lengths (loss_coef); NULL = e = 0 (scoring only)
+  int T, Bm, nb;
+  double alpha;
+  float* ent_out;    // [Bm*T] per-token H (through slot)
+};
+
 // one CTA per row
-__global__ void __launch_bounds__(1024)
-logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ targets,
-               const float* __restrict__ coef, const float* __restrict__ klw,
-               const float* __restrict__ ref_lp, const float* __restrict__ old_lp, float clip_eps,
-               float* __restrict__ lp_out, int V, int write_grad, const int* __restrict__ slot) {
-  __shared__ float red_m[32], red_s[32];
-  __shared__ float s_lse2, s_max2;
+template <bool ENT>
+__device__ __forceinline__ void logprob_row(bf16* __restrict__ logits, long long ld, const int* __restrict__ targets,
+                                            const float* __restrict__ coef, const float* __restrict__ klw,
+                                            const float* __restrict__ ref_lp, const float* __restrict__ old_lp,
+                                            float clip_eps, float* __restrict__ lp_out, int V, int write_grad,
+                                            const int* __restrict__ slot, const EntArgs& ea) {
+  __shared__ float red_m[32], red_s[32], red_u[32];
+  __shared__ float s_lse2, s_max2, s_ent;
   const size_t row = blockIdx.x;
   bf16* z = logits + row * ld;
   const bf16x8* zv = reinterpret_cast<const bf16x8*>(z);
   const int nvec = V / 8;  // V % 8 == 0 checked on host
   // ---- pass 1: online softmax statistics in the log2 domain ----
-  float m = -INFINITY, s = 0.f;
+  float m = -INFINITY, s = 0.f, u = 0.f;
   for (int i = threadIdx.x; i < nvec; i += blockDim.x) {
     float f[8];
     unpack8(zv[i], f);
@@ -41,18 +65,37 @@ logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ 
     for (int j = 1; j < 8; ++j) lm = fmaxf(lm, f[j]);
     lm *= LOG2E;
     if (lm > m) {
-      s *= exp2f(m - lm);
+      if constexpr (ENT) {
+        const float sc = exp2f(m - lm);
+        u = s > 0.f ? sc * (u + s * (m - lm)) : 0.f;
+        s *= sc;
+      } else {
+        s *= exp2f(m - lm);
+      }
       m = lm;
     }
 #pragma unroll
-    for (int j = 0; j < 8; ++j) s += exp2f(f[j] * LOG2E - m);
+    for (int j = 0; j < 8; ++j) {
+      if constexpr (ENT) {
+        const float d = f[j] * LOG2E - m;
+        const float ex = exp2f(d);
+        s += ex;
+        u += ex * d;
+      } else {
+        s += exp2f(f[j] * LOG2E - m);
+      }
+    }
   }
-  // warp then block combine of (m, s)
+  // warp then block combine of (m, s[, u])
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float om = __shfl_xor_sync(0xffffffffu, m, o);
     const float os = __shfl_xor_sync(0xffffffffu, s, o);
     const float nm = fmaxf(m, om);
+    if constexpr (ENT) {
+      const float ou = __shfl_xor_sync(0xffffffffu, u, o);
+      ent_combine(m, s, u, om, os, ou, nm);
+    }
     s = (nm == -INFINITY) ? 0.f : s * exp2f(m - nm) + os * exp2f(om - nm);
     m = nm;
   }
@@ -60,23 +103,30 @@ logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ 
   if (l == 0) {
     red_m[w] = m;
     red_s[w] = s;
+    if constexpr (ENT) red_u[w] = u;
   }
   __syncthreads();
   if (w == 0) {
     const int nw = blockDim.x >> 5;
     m = l < nw ? red_m[l] : -INFINITY;
     s = l < nw ? red_s[l] : 0.f;
+    if constexpr (ENT) u = l < nw ? red_u[l] : 0.f;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const float om = __shfl_xor_sync(0xffffffffu, m, o);
       const float os = __shfl_xor_sync(0xffffffffu, s, o);
       const float nm = fmaxf(m, om);
+      if constexpr (ENT) {
+        const float ou = __shfl_xor_sync(0xffffffffu, u, o);
+        ent_combine(m, s, u, om, os, ou, nm);
+      }
       s = (nm == -INFINITY) ? 0.f : s * exp2f(m - nm) + os * exp2f(om - nm);
       m = nm;
     }
     if (l == 0) {
       s_max2 = m;
       s_lse2 = m + log2f(s);  // log2-sum-exp2
+      if constexpr (ENT) s_ent = LN2 * (log2f(s) - u / s);
     }
   }
   __syncthreads();
@@ -101,11 +151,19 @@ logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ 
   // d k3 / d lp = 1 - exp(q - p); klw carries beta * mask / (len * Bm * nb)   (not in the reference: beta = 0)
   if (klw && ref_lp && klw[sl] != 0.f) c += klw[sl] * (1.f - __expf(ref_lp[sl] - lp));
   if (threadIdx.x == 0 && lp_out) lp_out[sl] = lp;
+  float H = 0.f, e = 0.f;
+  if constexpr (ENT) {
+    H = s_ent;
+    if (threadIdx.x == 0) ea.ent_out[sl] = H;
+    const int len = ea.lens ? ea.lens[sl / ea.T] : 0;
+    if (len > 0 && ea.mask[sl] != 0 && ea.alpha != 0.0)
+      e = (float)(ea.alpha / ((double)len * (double)ea.Bm * (double)ea.nb));
+  }
   if (!write_grad) return;
   __syncthreads();  // z[y] read above must precede the in-place overwrite
-  // ---- pass 2: dz = coef * (onehot - softmax), in place ----
+  // ---- pass 2: dz = coef * (onehot - softmax) [+ e p (ln p + H)], in place ----
   bf16x8* zw = reinterpret_cast<bf16x8*>(z);
-  if (c == 0.f) {
+  if (c == 0.f && (!ENT || e == 0.f)) {
     bf16x8 zero;
     zero.u = make_uint4(0u, 0u, 0u, 0u);
     for (int i = threadIdx.x; i < nvec; i += blockDim.x) zw[i] = zero;
@@ -117,11 +175,33 @@ logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ 
     const int base = i * 8;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-      const float p = exp2f(f[j] * LOG2E - lse2);
-      f[j] = c * (((base + j) == y ? 1.f : 0.f) - p);
+      if constexpr (ENT) {
+        const float t = f[j] * LOG2E - lse2;   // log2 p
+        const float p = exp2f(t);
+        f[j] = c * (((base + j) == y ? 1.f : 0.f) - p) + e * p * (t * LN2 + H);
+      } else {
+        const float p = exp2f(f[j] * LOG2E - lse2);
+        f[j] = c * (((base + j) == y ? 1.f : 0.f) - p);
+      }
     }
     zw[i] = pack8(f);
   }
+}
+
+__global__ void __launch_bounds__(1024)
+logprob_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ targets,
+               const float* __restrict__ coef, const float* __restrict__ klw,
+               const float* __restrict__ ref_lp, const float* __restrict__ old_lp, float clip_eps,
+               float* __restrict__ lp_out, int V, int write_grad, const int* __restrict__ slot) {
+  logprob_row<false>(logits, ld, targets, coef, klw, ref_lp, old_lp, clip_eps, lp_out, V, write_grad, slot, EntArgs{});
+}
+
+__global__ void __launch_bounds__(1024)
+logprob_entropy_kernel(bf16* __restrict__ logits, long long ld, const int* __restrict__ targets,
+                       const float* __restrict__ coef, const float* __restrict__ klw,
+                       const float* __restrict__ ref_lp, const float* __restrict__ old_lp, float clip_eps,
+                       float* __restrict__ lp_out, int V, int write_grad, const int* __restrict__ slot, EntArgs ea) {
+  logprob_row<true>(logits, ld, targets, coef, klw, ref_lp, old_lp, clip_eps, lp_out, V, write_grad, slot, ea);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -162,17 +242,24 @@ __global__ void loss_coef_kernel(const int* __restrict__ mask, const double* __r
 //   PG   (:375): loss_m = -(1/Bm) sum_i A_i * (sum_t mask*lp) / len_i
 //   GRPO (:467-470): importance = exp(lp - lp.detach()) == 1  =>  loss_m = -(1/Bm) sum_i A_i * [len_i>0]
 // The reference's returned scalar is the SUM of loss_m over micro-batches (quirk Q2) -> *accum += loss_m.
-__global__ void loss_value_kernel(const float* __restrict__ lp, const int* __restrict__ mask,
-                                  const double* __restrict__ adv, const float* __restrict__ ref_lp,
-                                  double beta, const float* __restrict__ old_lp, double clip_eps,
-                                  double* __restrict__ accum, int Bm, int T, int grpo) {
+// ENT: also L_H = -alpha (1/Bm) sum_i [len_i>0] (sum_t mask H) / len_i, and ent_accum[0] += sum mask*H,
+// ent_accum[1] += sum mask (single CTA, fixed order: deterministic).
+template <bool ENT>
+__device__ __forceinline__ void loss_value_body(const float* __restrict__ lp, const int* __restrict__ mask,
+                                                const double* __restrict__ adv, const float* __restrict__ ref_lp,
+                                                double beta, const float* __restrict__ old_lp, double clip_eps,
+                                                double* __restrict__ accum, int Bm, int T, int grpo,
+                                                const float* __restrict__ ent, double alpha,
+                                                double* __restrict__ ent_accum) {
   __shared__ double red[32];
-  double total = 0.0;
+  __shared__ double rede[32];
+  double total = 0.0, ent_sum = 0.0, ent_n = 0.0;
   for (int i = 0; i < Bm; ++i) {
-    double s = 0.0, kl = 0.0;
+    double s = 0.0, kl = 0.0, hs = 0.0;
     int cnt = 0;
     for (int t = threadIdx.x; t < T; t += blockDim.x) {
       if (mask[(size_t)i * T + t] != 0) {
+        if constexpr (ENT) hs += (double)ent[(size_t)i * T + t];
         const double p = (double)lp[(size_t)i * T + t];
         if (old_lp && clip_eps > 0.0) {   // clipped surrogate: s accumulates min(rho A, clip(rho) A) instead of lp
           const double rho = exp(p - (double)old_lp[(size_t)i * T + t]);
@@ -191,6 +278,7 @@ __global__ void loss_value_kernel(const float* __restrict__ lp, const int* __res
     }
     s = warp_sum_d(s);
     kl = warp_sum_d(kl);
+    if constexpr (ENT) hs = warp_sum_d(hs);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
     __syncthreads();
@@ -198,24 +286,52 @@ __global__ void loss_value_kernel(const float* __restrict__ lp, const int* __res
     if ((threadIdx.x & 31) == 0) {
       red[threadIdx.x >> 5] = s;
       redk[threadIdx.x >> 5] = kl;
+      if constexpr (ENT) rede[threadIdx.x >> 5] = hs;
     }
     __shared__ int redc[32];
     if ((threadIdx.x & 31) == 0) redc[threadIdx.x >> 5] = cnt;
     __syncthreads();
     if (threadIdx.x == 0) {
-      double ss = 0.0, kk = 0.0;
+      double ss = 0.0, kk = 0.0, hh = 0.0;
       int cc = 0;
       for (int w = 0; w < (blockDim.x >> 5); ++w) {
         ss += red[w];
         kk += redk[w];
         cc += redc[w];
+        if constexpr (ENT) hh += rede[w];
       }
       const bool clipped = old_lp && clip_eps > 0.0;
       if (cc > 0) total += (clipped ? ss / (double)cc : (grpo ? adv[i] : adv[i] * (ss / (double)cc))) - beta * (kk / (double)cc);
+      if constexpr (ENT) {
+        if (cc > 0 && alpha != 0.0) total += alpha * (hh / (double)cc);
+        ent_sum += hh;
+        ent_n += (double)cc;
+      }
     }
     __syncthreads();
   }
   if (threadIdx.x == 0) *accum += -total / (double)Bm;
+  if constexpr (ENT) {
+    if (threadIdx.x == 0 && ent_accum) {
+      ent_accum[0] += ent_sum;
+      ent_accum[1] += ent_n;
+    }
+  }
+}
+
+__global__ void loss_value_kernel(const float* __restrict__ lp, const int* __restrict__ mask,
+                                  const double* __restrict__ adv, const float* __restrict__ ref_lp,
+                                  double beta, const float* __restrict__ old_lp, double clip_eps,
+                                  double* __restrict__ accum, int Bm, int T, int grpo) {
+  loss_value_body<false>(lp, mask, adv, ref_lp, beta, old_lp, clip_eps, accum, Bm, T, grpo, nullptr, 0.0, nullptr);
+}
+
+__global__ void loss_value_entropy_kernel(const float* __restrict__ lp, const int* __restrict__ mask,
+                                          const double* __restrict__ adv, const float* __restrict__ ref_lp,
+                                          double beta, const float* __restrict__ old_lp, double clip_eps,
+                                          double* __restrict__ accum, int Bm, int T, int grpo,
+                                          const float* __restrict__ ent, double alpha, double* __restrict__ ent_accum) {
+  loss_value_body<true>(lp, mask, adv, ref_lp, beta, old_lp, clip_eps, accum, Bm, T, grpo, ent, alpha, ent_accum);
 }
 
 }  // namespace b200rl
@@ -308,6 +424,42 @@ extern "C" int b200rl_loss_value_clip(const float* lp, const int* mask, const do
                                       int grpo, void* stream) {
   B200RL_REQUIRE(lp && mask && adv && accum && Bm > 0 && T > 0, "loss_value: bad args");
   loss_value_kernel<<<1, 256, 0, STREAM>>>(lp, mask, adv, ref_lp, beta, old_lp, clip_eps, accum, Bm, T, grpo);
+  B200RL_LAUNCH_OK();
+  return 0;
+}
+
+// Per-token policy entropy and entropy bonus (reference: BaseLearner.compute_entropy_bonus, distributed_actor.py:266-281,
+// call sites commented out in the PG loss :377-379 and the GRPO loss :472-480).  Same arguments as b200rl_logprob_slots
+// plus: ent_out [Bm*T] f32 per-token H (required; addressed through slot), and the bonus weight
+// e = alpha * mask / (len * Bm * nb) derived from mask [Bm*T] and lens [Bm] (lens NULL or alpha 0: no bonus gradient).
+extern "C" int b200rl_logprob_entropy(void* logits, long long ld, const int* targets, const float* coef, const float* klw,
+                                      const float* ref_lp, const float* old_lp, double clip_eps, float* lp_out, int rows,
+                                      int V, int write_grad, const int* slot, const int* mask, const int* lens, int Bm,
+                                      int T, int nb, double alpha, float* ent_out, void* stream) {
+  B200RL_REQUIRE(logits && targets && rows > 0 && V > 0 && V % 8 == 0 && ld % 8 == 0,
+                 "logprob_entropy: bad args (rows=%d V=%d ld=%lld)", rows, V, ld);
+  B200RL_REQUIRE(!write_grad || coef, "logprob_entropy: write_grad needs coef");
+  B200RL_REQUIRE(clip_eps >= 0.0, "logprob_entropy: clip_eps must be >= 0");
+  B200RL_REQUIRE(ent_out && T > 0, "logprob_entropy: needs ent_out and T > 0");
+  B200RL_REQUIRE(alpha == 0.0 || !lens || (mask && Bm > 0 && nb > 0),
+                 "logprob_entropy: alpha != 0 with lens needs mask, Bm > 0 and nb > 0");
+  const int threads = V >= 8192 ? 1024 : 256;
+  EntArgs ea{mask, alpha != 0.0 ? lens : nullptr, T, Bm, nb, alpha, ent_out};
+  logprob_entropy_kernel<<<rows, threads, 0, STREAM>>>((bf16*)logits, ld, targets, coef, klw, ref_lp, old_lp,
+                                                       (float)clip_eps, lp_out, V, write_grad, slot, ea);
+  B200RL_LAUNCH_OK();
+  return 0;
+}
+
+// loss value with the entropy term (see loss_value_body); ent [Bm*T] = ent_out of b200rl_logprob_entropy,
+// ent_accum (device f64[2], optional) += {sum mask*H, sum mask}.
+extern "C" int b200rl_loss_value_entropy(const float* lp, const int* mask, const double* adv, const float* ref_lp,
+                                         double beta, const float* old_lp, double clip_eps, double* accum, int Bm, int T,
+                                         int grpo, const float* ent, double alpha, double* ent_accum, void* stream) {
+  B200RL_REQUIRE(lp && mask && adv && accum && Bm > 0 && T > 0, "loss_value_entropy: bad args");
+  B200RL_REQUIRE(ent, "loss_value_entropy: needs the per-token entropy");
+  loss_value_entropy_kernel<<<1, 256, 0, STREAM>>>(lp, mask, adv, ref_lp, beta, old_lp, clip_eps, accum, Bm, T, grpo, ent,
+                                                   alpha, ent_accum);
   B200RL_LAUNCH_OK();
   return 0;
 }

@@ -59,6 +59,10 @@ int b200rl_logprob_clip(void*, long long, const int*, const float*, const float*
 int b200rl_loss_value_clip(const float*, const int*, const double*, const float*, double, const float*, double, double*, int, int, int, void*);
 int b200rl_loss_coef_kl(const int*, const double*, float*, float*, double, int*, int, int, int, void*);
 int b200rl_loss_value_kl(const float*, const int*, const double*, const float*, double, double*, int, int, int, void*);
+int b200rl_logprob_entropy(void*, long long, const int*, const float*, const float*, const float*, const float*, double, float*,
+                           int, int, int, const int*, const int*, const int*, int, int, int, double, float*, void*);
+int b200rl_loss_value_entropy(const float*, const int*, const double*, const float*, double, const float*, double, double*, int,
+                              int, int, const float*, double, double*, void*);
 int b200rl_nf4_dequant(const void*, const float*, void*, int, int, int, void*);
 int b200rl_lora_pack(const float*, void*, const void*, int, int, void*);
 int b200rl_rope_pos(void*, const float*, const int*, int, long long, int, int, int, void*);
@@ -771,7 +775,7 @@ static int base_weight(b200rl_model* m, cudaStream_t st, int l, int which, const
 
 static int run_microbatch(b200rl_model* m, const Layout& lay, const double* adv, float* lp_out, double* loss_accum,
                           int nb, int grpo, int backward, int lora_off, const float* ref_lp, double kl_beta,
-                          const float* old_lp, double clip_eps, void* stream) {
+                          const float* old_lp, double clip_eps, const b200rl_entropy_args* ent, void* stream) {
   const b200rl_model_config& c = m->cfg;
   const b200rl_packed_batch* pb = lay.pb;
   const int M = lay.M, B = lay.B, T = lay.T, L = lay.L, P = lay.P;
@@ -786,6 +790,9 @@ static int run_microbatch(b200rl_model* m, const Layout& lay, const double* adv,
   const bool use_kl = backward && kl_beta != 0.0 && ref_lp;
   B200RL_REQUIRE(clip_eps >= 0.0, "model_microbatch: clip_eps must be >= 0");
   const bool use_clip = old_lp && clip_eps > 0.0;
+  // entropy (b200rl_entropy_args): per-token H whenever ent_out is given, the bonus term when alpha != 0
+  const bool use_ent = ent && (ent->ent_out || ent->alpha != 0.0 || ent->ent_accum);
+  B200RL_REQUIRE(!use_ent || ent->ent_out, "model_microbatch: entropy_alpha != 0 or ent_accum needs ent_out");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int H = c.hidden, I = c.inter, QKV = m->QKV, QD = m->QD, V = c.vocab;
   const long long Mt = c.max_tokens;
@@ -868,14 +875,27 @@ static int run_microbatch(b200rl_model* m, const Layout& lay, const double* adv,
   if (backward) RC(b200rl_loss_coef_kl(answer_mask, adv, m->coef, use_kl ? m->klw : nullptr, kl_beta, m->lens, B, T, nb, stream));
   float* lp = lp_out ? lp_out : m->lp;
   if (score_slot) B200RL_CUDA_OK(cudaMemsetAsync(lp, 0, sizeof(float) * (size_t)B * T, st));  // positions left out report 0
+  if (score_slot && use_ent) B200RL_CUDA_OK(cudaMemsetAsync(ent->ent_out, 0, sizeof(float) * (size_t)B * T, st));
   PM(CAT_LOGPROB, (backward ? 2.0 : 1.0) * R * V * 2);
-  RC(b200rl_logprob_slots(m->logits, V, targets, backward ? m->coef : nullptr, use_kl ? m->klw : nullptr,
-                          use_kl ? ref_lp : nullptr, use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, lp, R, V,
-                          backward ? 1 : 0, score_slot, stream));
+  if (use_ent)
+    RC(b200rl_logprob_entropy(m->logits, V, targets, backward ? m->coef : nullptr, use_kl ? m->klw : nullptr,
+                              use_kl ? ref_lp : nullptr, use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, lp, R, V,
+                              backward ? 1 : 0, score_slot, answer_mask, backward ? m->lens : nullptr, B, T, nb,
+                              backward ? ent->alpha : 0.0, ent->ent_out, stream));
+  else
+    RC(b200rl_logprob_slots(m->logits, V, targets, backward ? m->coef : nullptr, use_kl ? m->klw : nullptr,
+                            use_kl ? ref_lp : nullptr, use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, lp, R, V,
+                            backward ? 1 : 0, score_slot, stream));
   PM(CAT_MISC, 0);
-  if (loss_accum && adv)
-    RC(b200rl_loss_value_clip(lp, answer_mask, adv, use_kl ? ref_lp : nullptr, use_kl ? kl_beta : 0.0,
-                              use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, loss_accum, B, T, grpo, stream));
+  if (loss_accum && adv) {
+    if (use_ent)
+      RC(b200rl_loss_value_entropy(lp, answer_mask, adv, use_kl ? ref_lp : nullptr, use_kl ? kl_beta : 0.0,
+                                   use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, loss_accum, B, T, grpo,
+                                   ent->ent_out, ent->alpha, ent->ent_accum, stream));
+    else
+      RC(b200rl_loss_value_clip(lp, answer_mask, adv, use_kl ? ref_lp : nullptr, use_kl ? kl_beta : 0.0,
+                                use_clip ? old_lp : nullptr, use_clip ? clip_eps : 0.0, loss_accum, B, T, grpo, stream));
+  }
   if (!backward) {
     PM(CAT_END, 0);
     return 0;
@@ -1044,7 +1064,7 @@ extern "C" int b200rl_model_profile_read(b200rl_model* m, double* ms, double* wo
 static int classic_pass(b200rl_model* m, const int* ids, const int* attn_mask, const int* answer_mask, const double* adv,
                         float* lp_out, double* loss_accum, int B, int P, int T, int nb, int grpo, int backward,
                         int lora_off, const float* ref_lp, double kl_beta, const float* old_lp, double clip_eps,
-                        void* stream) {
+                        const b200rl_entropy_args* ent, void* stream) {
   B200RL_REQUIRE(m && ids && attn_mask && answer_mask, "model_microbatch: null pointer");
   const b200rl_model_config& c = m->cfg;
   const int L = P + T;
@@ -1054,7 +1074,8 @@ static int classic_pass(b200rl_model* m, const int* ids, const int* attn_mask, c
   Layout lay;
   lay.M = B * L; lay.B = B; lay.T = T; lay.L = L; lay.P = P;
   lay.ids = ids; lay.key_mask = attn_mask; lay.answer_mask = answer_mask; lay.pb = nullptr;
-  return run_microbatch(m, lay, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps, stream);
+  return run_microbatch(m, lay, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps, ent,
+                        stream);
 }
 
 extern "C" int b200rl_model_microbatch_ex(b200rl_model* m, const int* ids, const int* attn_mask,
@@ -1063,7 +1084,7 @@ extern "C" int b200rl_model_microbatch_ex(b200rl_model* m, const int* ids, const
                                           int backward, int lora_off, const float* ref_lp, double kl_beta,
                                           void* stream) {
   return classic_pass(m, ids, attn_mask, answer_mask, adv, lp_out, loss_accum, B, P, T, nb, grpo, backward, lora_off, ref_lp,
-                      kl_beta, nullptr, 0.0, stream);
+                      kl_beta, nullptr, 0.0, nullptr, stream);
 }
 
 extern "C" int b200rl_model_microbatch(b200rl_model* m, const int* ids, const int* attn_mask,
@@ -1076,7 +1097,8 @@ extern "C" int b200rl_model_microbatch(b200rl_model* m, const int* ids, const in
 
 static int packed_pass(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv, float* lp_out,
                        double* loss_accum, int nb, int grpo, int backward, int lora_off, const float* ref_lp,
-                       double kl_beta, const float* old_lp, double clip_eps, void* stream) {
+                       double kl_beta, const float* old_lp, double clip_eps, const b200rl_entropy_args* ent,
+                       void* stream) {
   B200RL_REQUIRE(m && pb, "model_microbatch_packed: null pointer");
   const b200rl_model_config& c = m->cfg;
   B200RL_REQUIRE(c.head_dim == 128, "model_microbatch_packed: the packed layout needs head_dim 128 (tcgen05 attention)");
@@ -1093,26 +1115,41 @@ static int packed_pass(b200rl_model* m, const b200rl_packed_batch* pb, const dou
   Layout lay;
   lay.M = pb->rows; lay.B = pb->B; lay.T = pb->T; lay.L = pb->max_pos; lay.P = 0;
   lay.ids = pb->ids; lay.key_mask = pb->key_mask; lay.answer_mask = pb->answer_mask; lay.pb = pb;
-  return run_microbatch(m, lay, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps, stream);
+  return run_microbatch(m, lay, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps, ent,
+                        stream);
 }
 
 extern "C" int b200rl_model_microbatch_packed(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv,
                                               float* lp_out, double* loss_accum, int nb, int grpo, int backward,
                                               int lora_off, const float* ref_lp, double kl_beta, void* stream) {
-  return packed_pass(m, pb, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, nullptr, 0.0, stream);
+  return packed_pass(m, pb, adv, lp_out, loss_accum, nb, grpo, backward, lora_off, ref_lp, kl_beta, nullptr, 0.0, nullptr,
+                     stream);
 }
 
 // general forms: the loss terms in one argument block (include/b200rl.h b200rl_loss_args)
 extern "C" int b200rl_model_pass(b200rl_model* m, const int* ids, const int* attn_mask, const int* answer_mask,
                                  const double* adv, float* lp_out, double* loss_accum, int B, int P, int T,
                                  const b200rl_loss_args* a, void* stream) {
-  B200RL_REQUIRE(a != nullptr, "model_pass: null args");
-  return classic_pass(m, ids, attn_mask, answer_mask, adv, lp_out, loss_accum, B, P, T, a->nb, a->grpo, a->backward,
-                      a->lora_off, a->ref_lp, a->kl_beta, a->old_lp, a->clip_eps, stream);
+  return b200rl_model_pass_ent(m, ids, attn_mask, answer_mask, adv, lp_out, loss_accum, B, P, T, a, nullptr, stream);
 }
 extern "C" int b200rl_model_pass_packed(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv, float* lp_out,
                                         double* loss_accum, const b200rl_loss_args* a, void* stream) {
+  return b200rl_model_pass_packed_ent(m, pb, adv, lp_out, loss_accum, a, nullptr, stream);
+}
+
+// with the per-token entropy / entropy bonus (reference: compute_entropy_bonus, distributed_actor.py:266-281; call sites
+// commented out at :377-379 and :472-480).  ent NULL = b200rl_model_pass / b200rl_model_pass_packed.
+extern "C" int b200rl_model_pass_ent(b200rl_model* m, const int* ids, const int* attn_mask, const int* answer_mask,
+                                     const double* adv, float* lp_out, double* loss_accum, int B, int P, int T,
+                                     const b200rl_loss_args* a, const b200rl_entropy_args* ent, void* stream) {
+  B200RL_REQUIRE(a != nullptr, "model_pass: null args");
+  return classic_pass(m, ids, attn_mask, answer_mask, adv, lp_out, loss_accum, B, P, T, a->nb, a->grpo, a->backward,
+                      a->lora_off, a->ref_lp, a->kl_beta, a->old_lp, a->clip_eps, ent, stream);
+}
+extern "C" int b200rl_model_pass_packed_ent(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv,
+                                            float* lp_out, double* loss_accum, const b200rl_loss_args* a,
+                                            const b200rl_entropy_args* ent, void* stream) {
   B200RL_REQUIRE(a != nullptr, "model_pass_packed: null args");
   return packed_pass(m, pb, adv, lp_out, loss_accum, a->nb, a->grpo, a->backward, a->lora_off, a->ref_lp, a->kl_beta,
-                     a->old_lp, a->clip_eps, stream);
+                     a->old_lp, a->clip_eps, ent, stream);
 }

@@ -78,6 +78,15 @@ class BaseLearner:
         self.clip_eps = float(config.get("clip_eps", 0.0))
         self.inner_epochs = max(1, int(config.get("inner_epochs", 1)))
         self.last_epoch_losses = []
+        # entropy bonus (reference: compute_entropy_bonus, distributed_actor.py:266-281, call sites commented out at
+        # :377-379 / :472-480, config key at :437): loss -= entropy_alpha * mean_i(sum_t mask H / len_i) per micro-batch, so
+        # alpha > 0 rewards entropy (DESIGN.md).  log_entropy: report the mean per-token entropy of the trained tokens in
+        # last_metrics(); implied by entropy_alpha != 0.
+        self.entropy_alpha = float(config.get("entropy_alpha", 0.0))
+        self.log_entropy = bool(config.get("log_entropy", False)) or self.entropy_alpha != 0.0
+        self._metrics = {}
+        self._ent_accum = torch.zeros(2, device=policy.device, dtype=torch.float64) if self.log_entropy else None
+        self._ent_buf = None
         # packed shared-prompt layout (packing.py): identical results, each distinct prompt of a micro-batch is
         # processed once; needs the tcgen05 attention kernels (head_dim 128)
         self.share_prompts = bool(config.get("share_prompts", policy.cfg.head_dim == 128))
@@ -120,19 +129,24 @@ class BaseLearner:
     def _h2d(self, t):
         return self._stager.to_device(t)
 
-    def compute_current_policy_probs(self, policy, messages, answers):
-        """(:215-261) -> (action_log_probs [B,T] fp32, answer_mask [B,T]) on the device; scoring only."""
+    def compute_current_policy_probs(self, policy, messages, answers, return_entropy=False):
+        """(:215-261) -> (action_log_probs [B,T] fp32, answer_mask [B,T]) on the device; scoring only.
+        return_entropy: (lp, mask, entropy [B,T] fp32 in nats), computed in the same pass over the logits."""
         ids, am, ansm = self._encode(messages, answers)
         B = ids.shape[0]
         lp = torch.empty(B, self.max_new_tokens, device=policy.device, dtype=torch.float32)
+        ekw = {}
+        if return_entropy:
+            ekw["ent_out"] = torch.empty(B, self.max_new_tokens, device=policy.device, dtype=torch.float32)
         if self.share_prompts:
             pk = self._pack(ids, am)
-            policy.microbatch_packed(pk, None, 1, False, backward=False, lp_out=lp)
-            return lp, pk.answer_mask
-        d_ansm = self._h2d(ansm)
-        policy.microbatch(self._h2d(ids), self._h2d(am), d_ansm, None, self.max_prompt_tokens,
-                          self.max_new_tokens, 1, False, backward=False, lp_out=lp)
-        return lp, d_ansm
+            policy.microbatch_packed(pk, None, 1, False, backward=False, lp_out=lp, **ekw)
+            mask = pk.answer_mask
+        else:
+            mask = self._h2d(ansm)
+            policy.microbatch(self._h2d(ids), self._h2d(am), mask, None, self.max_prompt_tokens,
+                              self.max_new_tokens, 1, False, backward=False, lp_out=lp, **ekw)
+        return (lp, mask, ekw["ent_out"]) if return_entropy else (lp, mask)
 
     def _pack(self, ids, am):
         host = packing.pack_microbatch(ids.numpy(), am.numpy(), self.max_prompt_tokens, self.max_new_tokens,
@@ -150,6 +164,11 @@ class BaseLearner:
         pol = self.policy
         pol.zero_grad()                                                       # :358 / :450
         pol.loss_accum.zero_()
+        ent_accum = self._ent_accum
+        if ent_accum is not None:
+            ent_accum.zero_()
+            if self._ent_buf is None:
+                self._ent_buf = torch.empty(pol.max_batch * self.max_new_tokens, device=pol.device, dtype=torch.float32)
         grpo = self.learner_type == "grpo"
         B = self.update_batch_size
         # plan the passes: runs of up to `fuse_microbatches` FULL micro-batches that survive the skip predicate
@@ -174,6 +193,10 @@ class BaseLearner:
             msgs, answ = [messages[j] for j in idx], [answers[j] for j in idx]
             r = rewards[idx] * float(k)          # see __init__: k fused micro-batches
             beta = self.kl_beta * k
+            ekw = {}
+            if ent_accum is not None:    # alpha scaled like the advantages and kl_beta (see __init__)
+                ekw = dict(entropy_alpha=self.entropy_alpha * k, ent_out=self._ent_buf[:len(idx) * self.max_new_tokens],
+                           ent_accum=ent_accum)
             ids, am, ansm = self._encode(msgs, answ)
             didx = torch.as_tensor(idx, device=pol.device) if (old_lp is not None or lp_capture is not None) else None
             olp = old_lp.index_select(0, didx).contiguous() if old_lp is not None else None
@@ -185,7 +208,7 @@ class BaseLearner:
                     ref_lp = torch.empty(len(idx), self.max_new_tokens, device=pol.device, dtype=torch.float32)
                     pol.microbatch_packed(pk, None, 1, False, backward=False, lp_out=ref_lp, lora_off=True)
                 pol.microbatch_packed(pk, self._h2d(torch.from_numpy(r)), nb, grpo, backward=True, ref_lp=ref_lp,
-                                      kl_beta=beta, lp_out=lp_now, old_lp=olp, clip_eps=clip)
+                                      kl_beta=beta, lp_out=lp_now, old_lp=olp, clip_eps=clip, **ekw)
             else:
                 d_ids, d_am, d_ansm = self._h2d(ids), self._h2d(am), self._h2d(ansm)
                 ref_lp = None
@@ -196,10 +219,20 @@ class BaseLearner:
                                    backward=False, lp_out=ref_lp, lora_off=True)
                 pol.microbatch(d_ids, d_am, d_ansm, self._h2d(torch.from_numpy(r)), self.max_prompt_tokens,
                                self.max_new_tokens, nb, grpo, backward=True, ref_lp=ref_lp, kl_beta=beta, lp_out=lp_now,
-                               old_lp=olp, clip_eps=clip)
+                               old_lp=olp, clip_eps=clip, **ekw)
             if lp_capture is not None:
                 lp_capture.index_copy_(0, didx, lp_now)
-        return float(pol.loss_accum.item())   # sum of per-micro-batch losses (quirk Q2), one sync
+        if ent_accum is None:
+            self._metrics = {}
+            return float(pol.loss_accum.item())   # sum of per-micro-batch losses (quirk Q2), one sync
+        loss, h_sum, n_tok = torch.cat([pol.loss_accum, ent_accum]).tolist()   # still one sync
+        self._metrics = {"entropy": h_sum / n_tok if n_tok > 0 else float("nan"), "entropy_tokens": int(n_tok)}
+        return loss
+
+    def last_metrics(self):
+        """Metrics of the last compute_loss / train / compute_gradients (first inner epoch): {"entropy": mean per-token
+        entropy in nats over the answer tokens trained, "entropy_tokens": their count}; {} when entropy logging is off."""
+        return dict(self._metrics)
 
     def _train_epochs(self, problems, answers, rewards):
         """One optimizer step per inner epoch on the same batch (reference: exactly one, :407-415 / :507-513).  Epoch 0 is
@@ -207,15 +240,19 @@ class BaseLearner:
         the clipped surrogate.  Returns the first epoch's loss (the number the reference returns)."""
         old = None
         self.last_epoch_losses = []
+        metrics = {}
         for epoch in range(self.inner_epochs):
             capture = None
             if epoch == 0 and self.inner_epochs > 1 and self.clip_eps > 0:
                 capture = torch.zeros(len(problems), self.max_new_tokens, device=self.policy.device, dtype=torch.float32)
             loss = self.compute_loss(problems, answers, rewards, old_lp=old, lp_capture=capture)
+            if epoch == 0:
+                metrics = self._metrics
             self.policy.optimizer_step(self.lr, weight_decay=self.weight_decay)
             self.last_epoch_losses.append(loss)
             if capture is not None:
                 old = capture
+        self._metrics = metrics
         return self.last_epoch_losses[0]
 
     # ---- gradient export / merge (:283-333) --------------------------------------------------------
@@ -302,10 +339,12 @@ class BaseLearner:
         process, one stream each — tests) must have launched every kernel once before the first P2P barrier spins on it."""
         pol = self.policy
         flat, m, v, step = pol.lora_flat.clone(), pol.adam_m.clone(), pol.adam_v.clone(), pol.opt_step
+        metrics = self._metrics
         B = min(self.update_batch_size, pol.max_batch)
         msgs = [[1, 2, 3]] * B
         answ = [[4, 5, 6, 7]] * B
-        self.compute_loss(msgs, answ, [1.0] * B)
+        self.compute_loss(msgs, answ, [1.0] * B)   # launches the entropy kernels too when they are enabled
+        self._metrics = metrics
         pol.optimizer_step(self.lr)
         pol.lora_flat.copy_(flat); pol.adam_m.copy_(m); pol.adam_v.copy_(v)
         pol.opt_step = step

@@ -160,6 +160,31 @@ def logprob(logits, targets, coef=None, write_grad=False):
     return lp
 
 
+def logprob_entropy(logits, targets, coef=None, write_grad=False, *, klw=None, ref_lp=None, old_lp=None, clip_eps=0.0,
+                    slot=None, mask=None, lens=None, T=None, Bm=0, nb=1, alpha=0.0, n_slots=None):
+    """logprob() plus the per-token entropy H = -sum p ln p of every row (b200rl_logprob_entropy).  Returns (lp, ent),
+    both [n_slots] (default: rows) and addressed through `slot` when given.  With write_grad and alpha != 0 the
+    gradient of the bonus -e*H, e = alpha * mask / (lens * Bm * nb) (mask [Bm*T], lens [Bm]), is added to dlogits."""
+    rows, V = logits.shape
+    n = n_slots if n_slots is not None else rows
+    lp = torch.zeros(n, device=logits.device, dtype=torch.float32)
+    ent = torch.zeros(n, device=logits.device, dtype=torch.float32)
+    check(lib().b200rl_logprob_entropy(ptr(logits), logits.stride(0), ptr(targets), ptr(coef), ptr(klw), ptr(ref_lp),
+                                       ptr(old_lp), float(clip_eps), ptr(lp), rows, V, 1 if write_grad else 0, ptr(slot),
+                                       ptr(mask), ptr(lens), int(Bm), int(T if T is not None else n), int(nb), float(alpha),
+                                       ptr(ent), stream()), "logprob_entropy")
+    return lp, ent
+
+
+def loss_value_entropy(lp, mask, adv, ent, alpha, accum, grpo, ent_accum=None):
+    """loss_value() plus the entropy term -alpha * mean_i(sum_t mask H / len_i); ent_accum f64[2] += {sum mask H, sum mask}."""
+    Bm, T = mask.shape
+    check(lib().b200rl_loss_value_entropy(ptr(lp), ptr(mask), ptr(adv), None, 0.0, None, 0.0, ptr(accum), Bm, T,
+                                          1 if grpo else 0, ptr(ent), float(alpha), ptr(ent_accum), stream()),
+          "loss_value_entropy")
+    return accum
+
+
 def loss_coef(mask, adv, nb):
     Bm, T = mask.shape
     coef = torch.empty(Bm, T, device=mask.device, dtype=torch.float32)

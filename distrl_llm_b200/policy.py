@@ -380,23 +380,42 @@ class Policy:
         return _capi.LossArgs(int(nb), 1 if grpo else 0, 1 if backward else 0, 1 if lora_off else 0, ptr(ref_lp),
                               float(kl_beta), ptr(old_lp), float(clip_eps))
 
+    @staticmethod
+    def _entropy_args(entropy_alpha, ent_out, ent_accum):
+        if not entropy_alpha and ent_out is None and ent_accum is None:
+            return None
+        return _capi.EntropyArgs(float(entropy_alpha), ptr(ent_out), ptr(ent_accum))
+
     def microbatch(self, ids, attn_mask, answer_mask, adv, P, T, nb, grpo, backward, lp_out=None,
-                   lora_off=False, ref_lp=None, kl_beta=0.0, old_lp=None, clip_eps=0.0):
+                   lora_off=False, ref_lp=None, kl_beta=0.0, old_lp=None, clip_eps=0.0, entropy_alpha=0.0, ent_out=None,
+                   ent_accum=None):
         """One micro-batch through the C++ driver. ids/attn_mask [B, P+T] int32, answer_mask [B,T] int32,
         adv [B] float64 (all on this device). Accumulates into lora_grad and self.loss_accum.
         lora_off: adapter-disabled scoring pass (reference policy); ref_lp + kl_beta: optional KL term;
-        old_lp [B,T] + clip_eps: optional clipped-ratio surrogate (b200rl_loss_args)."""
+        old_lp [B,T] + clip_eps: optional clipped-ratio surrogate (b200rl_loss_args);
+        ent_out [B,T] f32: per-token entropy; entropy_alpha: entropy bonus weight (needs ent_out); ent_accum f64[2]:
+        += {sum mask*H, sum mask} (b200rl_entropy_args)."""
         B = ids.shape[0]
         a = self._loss_args(nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps)
-        check(lib().b200rl_model_pass(self.handle, ptr(ids), ptr(attn_mask), ptr(answer_mask), ptr(adv), ptr(lp_out),
-                                      ptr(self.loss_accum), B, P, T, C.byref(a), stream()), "model_pass")
+        e = self._entropy_args(entropy_alpha, ent_out, ent_accum)
+        if e is None:
+            check(lib().b200rl_model_pass(self.handle, ptr(ids), ptr(attn_mask), ptr(answer_mask), ptr(adv), ptr(lp_out),
+                                          ptr(self.loss_accum), B, P, T, C.byref(a), stream()), "model_pass")
+            return
+        check(lib().b200rl_model_pass_ent(self.handle, ptr(ids), ptr(attn_mask), ptr(answer_mask), ptr(adv), ptr(lp_out),
+                                          ptr(self.loss_accum), B, P, T, C.byref(a), C.byref(e), stream()), "model_pass_ent")
 
     def microbatch_packed(self, packed, adv, nb, grpo, backward, lp_out=None, lora_off=False, ref_lp=None,
-                          kl_beta=0.0, old_lp=None, clip_eps=0.0):
+                          kl_beta=0.0, old_lp=None, clip_eps=0.0, entropy_alpha=0.0, ent_out=None, ent_accum=None):
         """Same as microbatch() on the packed shared-prompt layout (`packed`: packing.PackedDevice)."""
         a = self._loss_args(nb, grpo, backward, lora_off, ref_lp, kl_beta, old_lp, clip_eps)
-        check(lib().b200rl_model_pass_packed(self.handle, C.byref(packed.c), ptr(adv), ptr(lp_out), ptr(self.loss_accum),
-                                             C.byref(a), stream()), "model_pass_packed")
+        e = self._entropy_args(entropy_alpha, ent_out, ent_accum)
+        if e is None:
+            check(lib().b200rl_model_pass_packed(self.handle, C.byref(packed.c), ptr(adv), ptr(lp_out),
+                                                 ptr(self.loss_accum), C.byref(a), stream()), "model_pass_packed")
+            return
+        check(lib().b200rl_model_pass_packed_ent(self.handle, C.byref(packed.c), ptr(adv), ptr(lp_out), ptr(self.loss_accum),
+                                                 C.byref(a), C.byref(e), stream()), "model_pass_packed_ent")
 
     def debug_tensor(self, name, layer, shape, dtype=torch.bfloat16):
         p = lib().b200rl_model_debug_ptr(self.handle, name.encode(), layer)

@@ -5,6 +5,7 @@ Trainer and the actors read (:51-81).  Additions (all optional):
   --stub                 synthetic token-id dataset + StubGenerator actors + synthetic rewards (no dataset, tokenizer or vLLM
                          needed: this image has no network); implied by a `random:*` model
   --kl_beta / --clip_eps / --inner_epochs     KL-to-reference weight, clipped-ratio surrogate, epochs per batch (N4)
+  --entropy_alpha / --log_entropy   entropy bonus weight (> 0 rewards entropy) / log the mean per-token policy entropy
   --overlap_generation   generate batch k+1 while the learners train on batch k (N3)
   --adapter_sync         memory (default: device-to-device hand-off, N1) | file (PEFT directory like the reference)
   --max_steps, --bench   stop after that many trainer steps / print ONE JSON line with trainer steps per second
@@ -53,6 +54,8 @@ def build_parser():
     ap.add_argument("--kl_beta", type=float, default=0.0)
     ap.add_argument("--clip_eps", type=float, default=0.0)
     ap.add_argument("--inner_epochs", type=int, default=1)
+    ap.add_argument("--entropy_alpha", type=float, default=0.0)
+    ap.add_argument("--log_entropy", action="store_true")
     ap.add_argument("--overlap_generation", action="store_true")
     ap.add_argument("--adapter_sync", choices=["memory", "file"], default="memory")
     ap.add_argument("--fuse_microbatches", type=int, default=2)
@@ -71,6 +74,7 @@ def config_from_args(args):
         "actor_gpu_usage", "learner_gpu_usage", "lora_alpha", "lora_dropout")}
     cfg["use_vllm"] = True
     cfg.update(kl_beta=args.kl_beta, clip_eps=args.clip_eps, inner_epochs=args.inner_epochs,
+               entropy_alpha=args.entropy_alpha, log_entropy=args.log_entropy,
                overlap_generation=args.overlap_generation, adapter_sync=args.adapter_sync,
                fuse_microbatches=args.fuse_microbatches, max_steps=args.max_steps or None)
     return cfg

@@ -155,6 +155,16 @@ class Trainer:
 
     # ---- one policy update (reference :302-346) ---------------------------------------------------------------------
     def _update(self, candidates):
+        loss = self._update_learners(candidates)
+        self._update_metrics = {}
+        if self.config.get("log_entropy") or self.config.get("entropy_alpha", 0.0):
+            # token-weighted mean per-token policy entropy over every learner's trained tokens
+            ms = [m for m in _get([l.last_metrics.remote() for l in self.learners]) if m.get("entropy_tokens", 0) > 0]
+            n = sum(m["entropy_tokens"] for m in ms)
+            self._update_metrics["entropy"] = sum(m["entropy"] * m["entropy_tokens"] for m in ms) / n if n else float("nan")
+        return loss
+
+    def _update_learners(self, candidates):
         if self.num_learners == 1:
             return _get(self.learners[0].train.remote(candidates))
         problems, answers, rewards = self.merge_candidates(candidates)
@@ -206,6 +216,7 @@ class Trainer:
                 loss = self._update(candidates)
                 upd_s = time.time() - t0
                 self.save_adapter()
+                m.update(self._update_metrics)
                 m.update({"loss": loss, "episode": episode, "total_batch_steps": step, "total_samples_processed": samples,
                           "timing/update_duration": upd_s, "timing/reward_duration": rew_s, "timing/generation_duration": gen_s})
                 self._log(m, step)

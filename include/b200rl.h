@@ -168,6 +168,24 @@ int b200rl_logprob_slots(void* logits, long long ld, const int* targets, const f
 int b200rl_loss_value_clip(const float* lp, const int* mask, const double* adv, const float* ref_lp, double beta,
                            const float* old_lp, double clip_eps, double* accum, int Bm, int T, int grpo, void* stream);
 
+/* per-token policy entropy and entropy bonus (reference: BaseLearner.compute_entropy_bonus, distributed_actor.py:266-281,
+ * call sites commented out in the PG loss :377-379 and the GRPO loss :472-480).  Same as b200rl_logprob_slots, plus
+ *   ent_out [Bm*T] f32 (required): H = -sum_v p_v ln p_v of each scored row, p = softmax(z) at temperature 1, in nats,
+ *           written through slot like lp_out;
+ *   the bonus gradient e p_v (ln p_v + H) added to dlogits, e = alpha * mask / (len * Bm * nb) from mask [Bm*T] and
+ *           lens [Bm] (b200rl_loss_coef*); lens NULL or alpha 0 = no bonus.  alpha > 0 rewards entropy.
+ * lp_out is bit-identical to b200rl_logprob_slots'. */
+int b200rl_logprob_entropy(void* logits, long long ld, const int* targets, const float* coef, const float* klw,
+                           const float* ref_lp, const float* old_lp, double clip_eps, float* lp_out, int rows, int V,
+                           int write_grad, const int* slot, const int* mask, const int* lens, int Bm, int T, int nb,
+                           double alpha, float* ent_out, void* stream);
+/* b200rl_loss_value_clip plus L_H = -alpha (1/Bm) sum_i [len_i>0] (sum_t mask H) / len_i (reference :266-281, :377-379,
+ * :472-480); ent [Bm*T] = ent_out above; ent_accum (device f64[2], optional) += {sum mask*H, sum mask}.  One CTA,
+ * fixed summation order. */
+int b200rl_loss_value_entropy(const float* lp, const int* mask, const double* adv, const float* ref_lp, double beta,
+                              const float* old_lp, double clip_eps, double* accum, int Bm, int T, int grpo,
+                              const float* ent, double alpha, double* ent_accum, void* stream);
+
 /* ---- G9: group-relative advantages + top-k (distributed_trainer.py:262-294) ---------------- */
 int b200rl_group_advantage_topk(const double* rewards, double* values, double* baselines,
                                 int* topk_idx, double* topk_val, int G, int C, int k, int grpo,
@@ -317,6 +335,24 @@ int b200rl_model_pass(b200rl_model* m, const int* ids, const int* attn_mask, con
                       float* lp_out, double* loss_accum, int B, int P, int T, const b200rl_loss_args* args, void* stream);
 int b200rl_model_pass_packed(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv, float* lp_out,
                              double* loss_accum, const b200rl_loss_args* args, void* stream);
+/* Entropy of the policy and entropy bonus (reference: compute_entropy_bonus, distributed_actor.py:266-281; call sites
+ * commented out at :377-379 and :472-480; config key commented out at :437).
+ *   alpha      bonus weight: loss -= alpha * mean_i( sum_t mask H / len_i ) per micro-batch; > 0 rewards entropy
+ *   ent_out    [B*T] f32 device: per-token entropy in nats (0 for positions left out of compact scoring); required
+ *              whenever alpha != 0 or ent_accum is set
+ *   ent_accum  device f64[2] or NULL: += {sum mask*H, sum mask} of the pass (passes that compute a loss value only)
+ * args NULL in the calls below = b200rl_model_pass / b200rl_model_pass_packed. */
+typedef struct b200rl_entropy_args {
+  double alpha;
+  float* ent_out;
+  double* ent_accum;
+} b200rl_entropy_args;
+int b200rl_model_pass_ent(b200rl_model* m, const int* ids, const int* attn_mask, const int* answer_mask,
+                          const double* adv, float* lp_out, double* loss_accum, int B, int P, int T,
+                          const b200rl_loss_args* args, const b200rl_entropy_args* ent, void* stream);
+int b200rl_model_pass_packed_ent(b200rl_model* m, const b200rl_packed_batch* pb, const double* adv, float* lp_out,
+                                 double* loss_accum, const b200rl_loss_args* args, const b200rl_entropy_args* ent,
+                                 void* stream);
 
 /* per-op CUDA-event profiling of the driver (categories: 0 gemm, 1 skinny LoRA gemm, 2 dW gemm, 3 nf4
  * dequant, 4 attn fwd, 5 attn bwd, 6 row kernels, 7 logprob, 8 misc); read() returns sums since the last
